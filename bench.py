@@ -57,18 +57,80 @@ WORKLOAD = ('co-slam hash-grid(16 lvl x 2 feat, 2^16) + OneBlob16, 640x480 synth
             f'43 samples/ray, smoothness 31^3, {N_KEYFRAMES} keyframes')
 
 
+# --steps / --warmup when not given: the CPU ports of --impl reference take seconds per step
+DEFAULT_STEPS = {'ours': (200, 10), 'reference': (10, 2), 'reference_workload': (5, 0)}
+
+
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
-    ap.add_argument('--warmup', type=int, default=10)
+    ap.add_argument('--steps', type=int, default=None,
+                    help='timed steps (default 200; --impl reference: 10 for coslam, 5 otherwise)')
+    ap.add_argument('--warmup', type=int, default=None,
+                    help='untimed steps before them (default 10; --impl reference: 2 for coslam, '
+                         '0 otherwise)')
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--config', default='coslam', choices=['coslam', 'nice', 'vox', 'point'])
     ap.add_argument('--scaling', default='weak', choices=['weak', 'strong'],
                     help='N > 1: weak = fixed rays per GPU, strong = the single-GPU batch split over N')
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-torch-gpu-baseline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='write what the last timed step computed as DIR/<name>.npy (float32); '
+                         'default workload only (--impl ours --config coslam)')
+    args = ap.parse_args()
+    kind = args.impl if args.impl == 'ours' or args.config == 'coslam' else 'reference_workload'
+    steps, warmup = DEFAULT_STEPS[kind]
+    args.steps = steps if args.steps is None else args.steps
+    args.warmup = warmup if args.warmup is None else args.warmup
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and (args.impl != 'ours' or args.config != 'coslam'):
+        ap.error('--dump-outputs is implemented for the default workload '
+                 '(--impl ours --config coslam)')
+    return args
+
+
+DUMP_LIMIT = 64 * 1024 * 1024
+
+
+def dump_outputs(path, arrays):
+    """Write {name: tensor} as path/<name>.npy in float32 (float64 kept), at most DUMP_LIMIT
+    bytes in all, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy() if torch.is_tensor(t) else np.asarray(t)
+        a = a if a.dtype == np.float64 else a.astype(np.float32)
+        total += a.nbytes
+        if total > DUMP_LIMIT:
+            raise RuntimeError(f'--dump-outputs: more than {DUMP_LIMIT} bytes at {name}')
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
+def coslam_outputs(model, frames, sess, last):
+    """What one mapping iteration hands its caller: the loss and its terms, the per-ray
+    renders, and the parameters and poses after the optimiser step with the gradients they
+    were stepped with."""
+    out = {'loss': last['loss']}
+    if sess is not None:
+        renders = sess.out
+        out['loss_terms'] = torch.cat([sess.losses, sess.smooth_loss])
+        out['pose_rot'], out['pose_trans'] = sess.rot, sess.trans
+    else:
+        renders = last['out']
+        out['loss_terms'] = torch.stack([v.detach() for v in last['loss_dict'].values()])
+        out['pose_rot'] = torch.stack([f.pose.data_r.detach() for f in frames])
+        out['pose_trans'] = torch.stack([f.pose.data_t.detach() for f in frames])
+    for k, v in renders.items():
+        if torch.is_tensor(v) and v.is_floating_point():
+            out['render_' + k] = v
+    named = [('table', model.embed_fn.params)] + [
+        ('decoder_' + n.replace('.', '_'), p) for n, p in model.decoder.named_parameters()]
+    for n, p in named:
+        out[n] = p
+        out['grad_' + n] = p.grad
+    return out
 
 
 # ------------------------------------------------------------------ clocks ---
@@ -261,6 +323,8 @@ def run_ours(args):
         inp['smooth_rand'] = torch.rand(6)
         return inp
 
+    last = {}
+
     def device_step(inp):
         optim.zero_grad_all()
         out = model(inp)
@@ -269,6 +333,7 @@ def run_ours(args):
         loss.backward()
         allreduce_grads(dp)
         optim.optimizer_step_all(step=0)
+        last.update(out=out, loss_dict=loss_dict)
         return loss
 
     def barrier():
@@ -310,10 +375,12 @@ def run_ours(args):
     for i in range(K):
         flush.zero_()  # L2 flush (256 MB > 126 MB L2), outside the timed events
         ev[i][0].record()
-        run_step(W + i)
+        last['loss'] = run_step(W + i)
         ev[i][1].record()
     barrier()
     wall = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, coslam_outputs(model, frames, sess, last))
     ms = sum(a.elapsed_time(b) for a, b in ev)
     t = torch.tensor([ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -597,9 +664,8 @@ def run_reference(args):
     R = MAP_KF + MAP_CUR
     step = coslam_ref_step_factory(MAP_KF, MAP_CUR)
     cores = pick_threads(step)
-    K = min(args.steps, 10)
-    W = min(args.warmup, 2)
-    for _ in range(max(W, 1)):
+    K, W = args.steps, args.warmup
+    for _ in range(W):
         step()
     t0 = time.perf_counter()
     for _ in range(K):
@@ -786,7 +852,9 @@ def run_reference_workload(args):
         wl.build()  # the map (octree / point cloud) is built by the product's own maintenance code
     step, R, what = wl.cpu_step_factory()
     cores = pick_threads(step)
-    K = max(1, min(args.steps, 5))
+    K, W = args.steps, args.warmup
+    for _ in range(W):
+        step()
     t0 = time.perf_counter()
     for _ in range(K):
         step()
@@ -794,7 +862,7 @@ def run_reference_workload(args):
     v = R * K / dt
     print(json.dumps({
         'impl': 'reference', 'metric': wl.metric, 'value': v, 'unit': 'rays/s',
-        'n_gpus': int(os.environ.get('WORLD_SIZE', '1')), 'steps': K, 'warmup': 2,
+        'n_gpus': int(os.environ.get('WORLD_SIZE', '1')), 'steps': K, 'warmup': W,
         'ms_per_step': dt / K * 1e3, 'higher_is_better': True, 'scaling': 'weak',
         'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
         'config': {'workload': wl.workload, 'rays_per_step_per_gpu': R,

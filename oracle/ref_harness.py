@@ -1,9 +1,8 @@
 """Import the REAL reference classes from /root/reference (build container only).
 
-ORACLE / TEST INFRASTRUCTURE.  /root/reference does not exist on the GPU box, so
-everything here is used only (a) by tests marked ``needs_reference`` that pin the
-restated oracles against the reference's own Python, and (b) by
-tests/golden/make_golden.py which writes the committed fixtures.
+ORACLE / TEST INFRASTRUCTURE.  Used only by tests/golden/make_golden.py, which runs the
+reference's own Python and writes what the tests compare against into tests/golden/; the
+tests themselves never import the reference.
 
 The reference does not import cleanly under py3.12 (SURVEY.md section 0.4):
 non-arithmetic packages are replaced by MagicMock modules, ``tinycudann`` by the

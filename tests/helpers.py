@@ -1,8 +1,13 @@
 """Shared builders for the parity tests (oracle <-> CUDA path)."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import torch
 
 BOUND = np.array([[-3, 3], [-4, 2.5], [-2, 2.5]], dtype=np.float64)
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
 
 
 def make_rays(R, seed=0, zero_depth_every=7):
@@ -47,6 +52,20 @@ def coslam_pair(device, table_amp=0.3, seed=1, **cfg):
 
 def _t(x):
     return torch.from_numpy(np.asarray(x)) if not torch.is_tensor(x) else x
+
+
+def digest(x):
+    """SHA-256 of a tensor's dtype, shape and bytes: a bit-exact comparison against a stored
+    reference output without storing the output itself."""
+    t = _t(x).detach().cpu().contiguous()
+    h = hashlib.sha256(f'{t.dtype} {tuple(t.shape)} '.encode())
+    h.update(t.numpy().tobytes())
+    return h.hexdigest()
+
+
+def load_golden_json(name):
+    with open(os.path.join(GOLDEN, name)) as f:
+        return json.load(f)
 
 
 def rel_err(a, b):
@@ -142,10 +161,13 @@ def nice_from_golden(g, kind, device=None):
 
 
 def load_golden_pointslam():
-    import os
-    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden',
-                             'pointslam_geo_step.npz'))
-    return {k: g[k] for k in g.files}
+    """Inputs + stage 'geometry' (pointslam_geo_step.npz) and stage 'color' outputs
+    (pointslam_color_step.npz, keys cmap.* / ctrk.*)."""
+    out = {}
+    for name in ('pointslam_geo_step.npz', 'pointslam_color_step.npz'):
+        g = np.load(os.path.join(GOLDEN, name))
+        out.update({k: g[k] for k in g.files})
+    return out
 
 
 def pointslam_from_golden(g, kind, device=None):

@@ -1,5 +1,5 @@
-"""CPU tests (no GPU): the oracle is pinned to the reference's own classes and to the
-committed golden vectors; the C-ABI library loads and exports every declared symbol."""
+"""CPU tests (no GPU): the oracle is pinned to the reference's own classes through the
+committed golden vectors and digests (tests/golden/make_golden.py); the C-ABI library loads and exports every declared symbol."""
 import ctypes as C
 import os
 import re
@@ -8,8 +8,8 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import (BOUND, load_golden_coslam, make_rays, max_abs, rel_err,
-                     set_coslam_params)
+from helpers import (BOUND, digest, load_golden_coslam, load_golden_json, make_rays, max_abs,
+                     rel_err, set_coslam_params)
 
 
 def _oracle_from_golden():
@@ -43,47 +43,45 @@ def test_oracle_matches_golden_reference_vectors():
     assert int((ora.embed_fn.params.grad != 0).sum()) == int(g['d_table_nnz'])
 
 
-@pytest.mark.needs_reference
-def test_oracle_matches_reference_class_live():
-    """Run the reference's JointEncoding (from /root/reference) beside the oracle."""
-    from oracle import ref_harness
+def coslam_live_case():
+    """Oracle with seeded parameters (table x 3000 of the reference's init scale: non-trivial
+    sdf sign changes), rays and the noise the reference draws after torch.manual_seed(9)."""
     from oracle.coslam import CoslamOracle
-    bb = torch.from_numpy(BOUND)
-    ref = ref_harness.ref_joint_encoding(bb)
     ora = CoslamOracle(BOUND)
+    g = torch.Generator().manual_seed(21)
     with torch.no_grad():
-        ora.embed_fn.params.copy_(ref.embed_fn.params)
-        ora.sdf0.weight.copy_(ref.decoder.sdf_net.model[0].weight)
-        ora.sdf1.weight.copy_(ref.decoder.sdf_net.model[2].weight)
-        ora.col0.weight.copy_(ref.decoder.color_net.model[0].weight)
-        ora.col1.weight.copy_(ref.decoder.color_net.model[2].weight)
-        ref.embed_fn.params.mul_(3000.0)   # non-trivial sdf sign changes
-        ora.embed_fn.params.mul_(3000.0)
+        ora.embed_fn.params.copy_((torch.rand(ora.embed_fn.params.shape, generator=g) * 2 - 1) * 0.3)
+        for lin in (ora.sdf0, ora.sdf1, ora.col0, ora.col1):
+            lin.weight.copy_(torch.randn(lin.weight.shape, generator=g) / np.sqrt(lin.weight.shape[1]))
     R = 80
     rays_o, rays_d, ts, td, _ = make_rays(R, seed=3)
     torch.manual_seed(9)
     noise = torch.rand(R, 43)
     r1, r2 = torch.rand(3), torch.rand((1, 1, 1, 3))
-    torch.manual_seed(9)
-    inp = dict(rays_o=rays_o, rays_d=rays_d, target_s=ts, target_d=td, first=False)
-    out_r = ref(inp)
-    ld_r = ref.get_loss_dict(out_r, inp, True, 0)
-    out_o, ld_o, _ = ora.step(rays_o, rays_d, ts, td, noise, True, False,
-                              smooth_rand=torch.stack([r1, r2.reshape(3)]))
-    for k in ('rgb', 'depth', 'z_vals', 'raw', 'depth_var', 'disp_map', 'acc_map'):
-        assert torch.equal(out_r[k], out_o[k]), k
-    for k in ld_r:
-        assert float(ld_r[k]) == float(ld_o[k]), k
-    # render-only path (target_d=None -> 256 uniform samples)
     torch.manual_seed(4)
     n256 = torch.rand(R, 256)
-    torch.manual_seed(4)
-    o2 = ref(dict(rays_o=rays_o, rays_d=rays_d, target_s=None, target_d=None))
+    return ora, (rays_o, rays_d, ts, td), noise, torch.stack([r1, r2.reshape(3)]), n256
+
+
+COSLAM_OUT_KEYS = ('rgb', 'depth', 'z_vals', 'raw', 'depth_var', 'disp_map', 'acc_map')
+
+
+def test_oracle_matches_reference_class_live(one_thread):
+    """The reference's JointEncoding on the same parameters, rays and noise: outputs and losses
+    bit-identical (tests/golden/reference_cpu.json, written by make_golden.py reference_cpu)."""
+    g = load_golden_json('reference_cpu.json')['coslam']
+    ora, (rays_o, rays_d, ts, td), noise, smooth_rand, n256 = coslam_live_case()
+    out_o, ld_o, _ = ora.step(rays_o, rays_d, ts, td, noise, True, False, smooth_rand=smooth_rand)
+    for k in COSLAM_OUT_KEYS:
+        assert digest(out_o[k]) == g['out'][k], k
+    assert set(ld_o) == set(g['losses'])
+    for k in ld_o:
+        assert float(ld_o[k].detach()) == g['losses'][k], k
+    # render-only path (target_d=None -> 256 uniform samples)
     o3 = ora.render_rays(rays_o, rays_d, None, n256)
-    assert torch.equal(o2['rgb'], o3['rgb']) and torch.equal(o2['depth'], o3['depth'])
+    assert digest(o3['rgb']) == g['render']['rgb'] and digest(o3['depth']) == g['render']['depth']
 
 
-@pytest.mark.needs_reference
 def test_pose_roundtrip_like_frame_assert():
     """slam/common/frame.py:40-43: |pose - from_matrix(pose).matrix()| < 1e-3, for the
     matrix the reference's own __main__ check uses (opt_pose.py:112-124)."""
@@ -210,102 +208,98 @@ def test_nice_oracle_matches_golden_reference_vectors():
             <= 1e-6 * float(g[tag + '.d_grid_color_norm'])
 
 
-@pytest.mark.needs_reference
-def test_nice_oracle_coarse_stage_matches_reference_class_live():
-    """Stage 'coarse' (MLP_no_xyz on the 2 m grid over the doubled bound, 32 uniform samples,
-    no depth guidance): the reference's own ConvOnet(coarse=True) vs oracle/nice.py, outputs,
-    loss and the coarse-grid gradient bit-identical."""
-    from oracle import ref_harness
-    from oracle.nice import NiceOracle
-    bound = np.array([[-2.0, 2.0], [-2.5, 2.0], [-2.0, 2.3]])
-    torch.manual_seed(3)
-    ref = ref_harness.ref_conv_onet(bound, coarse=True)
-    ora = NiceOracle(bound, coarse=True)
-    ref_harness.copy_nice_ref_to_oracle(ref, ora)
-    assert tuple(ref.grid_c['grid_coarse'].shape) == tuple(ora.grids['grid_coarse'].shape)
-    with torch.no_grad():
-        ora.grids['grid_coarse'].mul_(30)
-        ref.grid_c['grid_coarse'] = ref.grid_c['grid_coarse'] * 30
-        for lin in list(ora.coarse.pts) + [ora.coarse.out]:
-            lin.bias.add_(0.05)
-        for i in range(5):
-            ref.decoder.coarse_decoder.pts_linears[i].bias.add_(0.05)
-        ref.decoder.coarse_decoder.output_linear.bias.add_(0.05)
-    ref.grid_c['grid_coarse'].requires_grad_(True)
-    assert torch.equal(ref.decoder.coarse_decoder.bound, ora.coarse_bound)
-    g = torch.Generator().manual_seed(4)
-    R = 50
+NICE_COARSE_BOUND = np.array([[-2.0, 2.0], [-2.5, 2.0], [-2.0, 2.3]])
+NICE_BOUND = np.array([[-2.0, 2.0], [-2.0, 2.0], [-2.0, 2.0]])
+OFFICE0_BOUND = np.array([[-5.5, 5.9], [-6.7, 5.4], [-4.7, 5.3]])
+
+
+def _nice_rays(R, seed):
+    g = torch.Generator().manual_seed(seed)
     rays_o = (torch.rand(R, 3, generator=g) - 0.5) * 0.5
     rays_d = torch.nn.functional.normalize(torch.randn(R, 3, generator=g), dim=-1)
     td = torch.rand(R, 1, generator=g) * 1.5 + 0.3
     td[3::7] = 0
     ts = torch.rand(R, 3, generator=g)
-    inp = dict(rays_o=rays_o, rays_d=rays_d, target_s=ts, target_d=td, stage='coarse')
-    with ref_harness.cuda_calls_are_noops():
-        out_r = ref(inp)
-    out_o = ora.render(rays_o, rays_d, td, 'coarse')
-    assert out_o['z_vals'].shape == (R, 32)
-    for k in ('depth', 'uncertainty'):
-        assert torch.equal(out_r[k], out_o[k]), k
-    ld_r = ref.get_loss_dict(out_r, inp, True, 'coarse')
-    ld_o = ora.loss_dict(out_o, ts, td, True, 'coarse')
-    assert set(ld_r) == set(ld_o) == {'depth_loss'}
-    assert float(ld_r['depth_loss'].detach()) == float(ld_o['depth_loss'].detach())
-    ld_r['depth_loss'].backward()
-    ld_o['depth_loss'].backward()
-    assert torch.equal(ref.grid_c['grid_coarse'].grad, ora.grids['grid_coarse'].grad)
+    return rays_o, rays_d, ts, td
 
 
-@pytest.mark.needs_reference
-def test_nice_oracle_matches_reference_class_live():
-    from oracle import ref_harness
+def nice_coarse_case():
+    """Seeded oracle with the coarse level: coarse grid x 30 and biases + 0.05 (non-trivial
+    occupancies), 50 rays."""
     from oracle.nice import NiceOracle
-    bound = np.array([[-2.0, 2.0], [-2.0, 2.0], [-2.0, 2.0]])
-    torch.manual_seed(1)
-    ref = ref_harness.ref_conv_onet(bound)
-    ora = NiceOracle(bound)
-    ref_harness.copy_nice_ref_to_oracle(ref, ora)
+    torch.manual_seed(3)  # fc_c layers keep torch's default init
+    ora = NiceOracle(NICE_COARSE_BOUND, coarse=True, seed=3)
+    with torch.no_grad():
+        ora.grids['grid_coarse'].mul_(30)
+        for lin in list(ora.coarse.pts) + [ora.coarse.out]:
+            lin.bias.add_(0.05)
+    return ora, _nice_rays(50, 4)
+
+
+def test_nice_oracle_coarse_stage_matches_reference_class_live(one_thread):
+    """Stage 'coarse' (MLP_no_xyz on the 2 m grid over the doubled bound, 32 uniform samples,
+    no depth guidance): the reference's own ConvOnet(coarse=True) on the same parameters vs
+    oracle/nice.py, outputs, loss and the coarse-grid gradient bit-identical."""
+    g = load_golden_json('reference_cpu.json')['nice_coarse']
+    ora, (rays_o, rays_d, ts, td) = nice_coarse_case()
+    assert list(ora.grids['grid_coarse'].shape) == g['grid_coarse_shape']
+    assert digest(ora.coarse_bound) == g['coarse_bound']
+    out_o = ora.render(rays_o, rays_d, td, 'coarse')
+    assert out_o['z_vals'].shape == (50, 32)
+    for k in ('depth', 'uncertainty'):
+        assert digest(out_o[k]) == g['out'][k], k
+    ld_o = ora.loss_dict(out_o, ts, td, True, 'coarse')
+    assert set(ld_o) == {'depth_loss'}
+    assert float(ld_o['depth_loss'].detach()) == g['depth_loss']
+    ld_o['depth_loss'].backward()
+    assert digest(ora.grids['grid_coarse'].grad) == g['d_grid_coarse']
+
+
+def nice_case():
+    """Seeded oracle, grids x 30 (non-trivial occupancies), 64 rays."""
+    from oracle.nice import NiceOracle
+    torch.manual_seed(1)  # fc_c layers keep torch's default init
+    ora = NiceOracle(NICE_BOUND, seed=1)
     with torch.no_grad():
         for k in ora.grids:
             ora.grids[k].mul_(30)
-            ref.grid_c[k] = ref.grid_c[k] * 30
-    assert torch.equal(ref.bounding_box, ora.bound)
-    g = torch.Generator().manual_seed(2)
-    R = 64
-    rays_o = (torch.rand(R, 3, generator=g) - 0.5) * 0.5
-    rays_d = torch.nn.functional.normalize(torch.randn(R, 3, generator=g), dim=-1)
-    td = torch.rand(R, 1, generator=g) * 1.5 + 0.3
-    td[3::7] = 0
-    ts = torch.rand(R, 3, generator=g)
-    inp = dict(rays_o=rays_o, rays_d=rays_d, target_s=ts, target_d=td, stage='color')
-    out_r = ref(inp)
+    return ora, _nice_rays(64, 2)
+
+
+def test_nice_oracle_matches_reference_class_live(one_thread):
+    """The reference's ConvOnet on the same parameters: stages color, middle and fine,
+    outputs and mapping / tracking losses bit-identical."""
+    from oracle.nice import NiceOracle
+    g = load_golden_json('reference_cpu.json')['nice']
+    ora, (rays_o, rays_d, ts, td) = nice_case()
+    assert digest(ora.bound) == g['bound']
     out_o = ora.render(rays_o, rays_d, td, 'color')
     for k in ('rgb', 'depth', 'uncertainty'):
-        assert torch.equal(out_r[k], out_o[k]), k
+        assert digest(out_o[k]) == g['color']['out'][k], k
     for m in (True, False):
-        ld_r = ref.get_loss_dict(out_r, inp, m, 'color')
         ld_o = ora.loss_dict(out_o, ts, td, m, 'color')
-        for k in ld_r:
-            assert float(ld_r[k].detach()) == float(ld_o[k].detach()), (m, k)
+        ref = g['color']['losses'][str(m)]
+        assert set(ld_o) == set(ref)
+        for k in ld_o:
+            assert float(ld_o[k].detach()) == ref[k], (m, k)
     # stages middle / fine are CUDA-only in the reference (Q5: device = f'cuda:{p.get_device()}');
-    # with that string neutralised the reference's own class runs them on the host
-    with ref_harness.cuda_calls_are_noops():
-        for stage in ('middle', 'fine'):
-            inp_s = dict(inp, stage=stage)
-            out_r = ref(inp_s)
-            out_o = ora.render(rays_o, rays_d, td, stage)
-            for k in ('depth', 'uncertainty'):
-                assert torch.equal(out_r[k], out_o[k]), (stage, k)
-            for m in (True, False):
-                ld_r = ref.get_loss_dict(out_r, inp_s, m, stage)
-                ld_o = ora.loss_dict(out_o, ts, td, m, stage)
-                assert set(ld_r) == set(ld_o)
-                for k in ld_r:
-                    assert float(ld_r[k].detach()) == float(ld_o[k].detach()), (stage, m, k)
+    # the stored values come from its own class run on the host with that string neutralised
+    for stage in ('middle', 'fine'):
+        out_o = ora.render(rays_o, rays_d, td, stage)
+        for k in ('depth', 'uncertainty'):
+            assert digest(out_o[k]) == g[stage]['out'][k], (stage, k)
+        for m in (True, False):
+            ld_o = ora.loss_dict(out_o, ts, td, m, stage)
+            ref = g[stage]['losses'][str(m)]
+            assert set(ld_o) == set(ref)
+            for k in ld_o:
+                assert float(ld_o[k].detach()) == ref[k], (stage, m, k)
     # the reference's grid-shape hazard (SURVEY Q2) at the default office0 bound
-    ref2 = ref_harness.ref_conv_onet(np.array([[-5.5, 5.9], [-6.7, 5.4], [-4.7, 5.3]]))
-    assert tuple(ref2.grid_c['grid_middle'].shape) == (1, 32, 31, 37, 35)
-    assert tuple(ref2.grid_c['grid_fine'].shape) == (1, 32, 63, 75, 71)
+    assert g['office0_shapes'] == {'grid_middle': [1, 32, 31, 37, 35],
+                                   'grid_fine': [1, 32, 63, 75, 71]}
+    o2 = NiceOracle(OFFICE0_BOUND)
+    for k, shp in g['office0_shapes'].items():
+        assert list(o2.grids[k].shape) == shp, k
 
 
 @pytest.mark.parametrize('tag,is_mapping', [('map', True), ('trk', False)])
@@ -473,86 +467,57 @@ def test_keyframe_selection_overlap_on_host():
     assert len(keyframe_selection_overlap(cam, frames[0], frames[1:], k=1, device='cpu')) == 1
 
 
-@pytest.mark.needs_reference
-def test_host_frontend_bit_identical_to_reference_functions():
+FRONTEND_KW = (dict(Hedge=0, Wedge=0), dict(Hedge=7, Wedge=11),
+               dict(Hedge=3, Wedge=5, depth_filter=True, return_index=True))
+
+
+def test_host_frontend_bit_identical_to_reference_functions(one_thread):
     """common.get_samples / get_rays / get_camera_rays (host tensors) against the reference's
     own slam.common.common / slam.utils.utils functions under the same torch seed: identical
     pixel draws, rays, depth / colour gathers and index outputs (rows A1-A5)."""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip('needs /root/reference')
-    ref_harness.install()
-    import slam.common.common as rc
-    import slam.utils.utils as ru
-    from slam.common.camera import Camera as RCam
     import xrdslam_b200.common as mc
     from xrdslam_b200.synthetic import make_sequence
+    g = load_golden_json('reference_cpu.json')['frontend']
     cam, poses, fr = make_sequence(1, width=160, height=120)
-    rcam = RCam(cam.fx, cam.fy, cam.cx, cam.cy, cam.width, cam.height)
     c2w = torch.from_numpy(poses[0])
     rgb, depth = fr[0]
-    for kw in (dict(Hedge=0, Wedge=0), dict(Hedge=7, Wedge=11),
-               dict(Hedge=3, Wedge=5, depth_filter=True, return_index=True)):
-        torch.manual_seed(5)
-        a = rc.get_samples(rcam, 333, c2w, depth, rgb, device='cpu', **kw)
+    for kw, ref in zip(FRONTEND_KW, g['get_samples']):
         torch.manual_seed(5)
         b = mc.get_samples(cam, 333, c2w, depth, rgb, device='cpu', **kw)
-        assert len(a) == len(b)
-        for x, y in zip(a, b):
-            assert x.dtype == y.dtype and torch.equal(x, y), kw
-    for x, y in zip(rc.get_rays(rcam, c2w, 'cpu'), mc.get_rays(cam, c2w, 'cpu')):
-        assert torch.equal(x, y)
-    assert torch.equal(torch.as_tensor(ru.get_camera_rays(120, 160, cam.fx, cam.fy, cam.cx, cam.cy)),
-                       mc.get_camera_rays(120, 160, cam.fx, cam.fy, cam.cx, cam.cy))
+        assert [digest(y) for y in b] == ref, kw
+    assert [digest(y) for y in mc.get_rays(cam, c2w, 'cpu')] == g['get_rays']
+    assert digest(mc.get_camera_rays(120, 160, cam.fx, cam.fy, cam.cx, cam.cy)) == g['get_camera_rays']
 
 
-@pytest.mark.needs_reference
+def optimizers_case(mod):
+    A = mod.AdamOptimizerConfig
+    torch.manual_seed(0)
+    p = {'a': [torch.nn.Parameter(torch.randn(5))], 'pose': [torch.nn.Parameter(torch.randn(3))]}
+    cfg = {'a': {'optimizer': A(lr=1e-2, weight_decay=1e-6, betas=(0.9, 0.99)), 'scheduler': None},
+           'pose': {'optimizer': A(lr=1e-3, accum_step=5), 'scheduler': None}}
+    opt = mod.Optimizers(cfg, p)
+    g = torch.Generator().manual_seed(1)
+    for step in range(12):
+        opt.zero_grad_all()
+        for k in p:
+            gr = torch.randn(p[k][0].shape, generator=g)
+            p[k][0].grad = gr if p[k][0].grad is None else p[k][0].grad + gr
+        opt.optimizer_step_all(step=step)
+    return {k: digest(v[0]) for k, v in p.items()}
+
+
 def test_optimizers_match_reference_engine_incl_accum_step():
     """xrdslam_b200.optimizers.Optimizers (zero_grad_all / optimizer_step_all, accum_step = 5,
     weight decay, custom betas) against the reference's own slam.engine.optimizers on host
     parameters: bit-identical after 12 steps (rows B2 / B3, Q11)."""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip('needs /root/reference')
-    ref_harness.install()
-    import slam.engine.optimizers as ro
     import xrdslam_b200.optimizers as mo
-
-    def run(mod):
-        A = mod.AdamOptimizerConfig
-        torch.manual_seed(0)
-        p = {'a': [torch.nn.Parameter(torch.randn(5))], 'pose': [torch.nn.Parameter(torch.randn(3))]}
-        cfg = {'a': {'optimizer': A(lr=1e-2, weight_decay=1e-6, betas=(0.9, 0.99)), 'scheduler': None},
-               'pose': {'optimizer': A(lr=1e-3, accum_step=5), 'scheduler': None}}
-        opt = mod.Optimizers(cfg, p)
-        g = torch.Generator().manual_seed(1)
-        for step in range(12):
-            opt.zero_grad_all()
-            for k in p:
-                gr = torch.randn(p[k][0].shape, generator=g)
-                p[k][0].grad = gr if p[k][0].grad is None else p[k][0].grad + gr
-            opt.optimizer_step_all(step=step)
-        return {k: v[0].detach().clone() for k, v in p.items()}
-    a, b = run(ro), run(mo)
-    for k in a:
-        assert torch.equal(a[k], b[k]), k
+    assert optimizers_case(mo) == load_golden_json('reference_cpu.json')['optimizers']
 
 
-@pytest.mark.needs_reference
-def test_keyframe_selection_overlap_matches_reference_function():
-    """Same seeds -> the same keyframes in the same order as the reference's own
-    slam.common.common.keyframe_selection_overlap (host tensors)."""
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip('needs /root/reference')
-    ref_harness.install()
-    import slam.common.common as rc
-    from slam.common.camera import Camera as RCam
+def keyframe_case():
     from xrdslam_b200.frame import Frame
-    from xrdslam_b200.keyframe_selection import keyframe_selection_overlap
     from xrdslam_b200.synthetic import CENTRE, look_at, make_camera, render_frame
     cam = make_camera(160, 120)
-    rcam = RCam(cam.fx, cam.fy, cam.cx, cam.cy, cam.width, cam.height)
     eye = CENTRE + np.array([0.5, 0.0, 0.1])
     tgt = CENTRE + np.array([-1.5, 0.3, -0.2])
     rng = np.random.default_rng(0)
@@ -562,14 +527,20 @@ def test_keyframe_selection_overlap_matches_reference_function():
     for k, p in enumerate(poses):
         rgb, depth = render_frame(cam, p, seed=k)
         frames.append(Frame(k, rgb, depth, init_pose=p, rot_rep='quat'))
+    return cam, frames
+
+
+def test_keyframe_selection_overlap_matches_reference_function():
+    """Same seeds -> the same keyframes in the same order as the reference's own
+    slam.common.common.keyframe_selection_overlap (host tensors)."""
+    from xrdslam_b200.keyframe_selection import keyframe_selection_overlap
+    g = load_golden_json('reference_cpu.json')['keyframes']
+    cam, frames = keyframe_case()
     for k in (2, 4, 8):
         torch.manual_seed(3)
         np.random.seed(3)
-        a = rc.keyframe_selection_overlap(rcam, frames[0], frames[1:], k, device='cpu')
-        torch.manual_seed(3)
-        np.random.seed(3)
         b = keyframe_selection_overlap(cam, frames[0], frames[1:], k, device='cpu')
-        assert [f.fid for f in a] == [f.fid for f in b], k
+        assert [f.fid for f in b] == g[str(k)], k
     assert 8 not in [f.fid for f in b]  # the frame looking the other way has no overlap
 
 
@@ -608,45 +579,30 @@ def test_convonet_load_pretrain_key_mapping(tmp_path):
             camera=cam, bounding_box=bound)
 
 
-@pytest.mark.needs_reference
-def test_pixel_grad_sampler_bit_identical_to_reference_function():
+PIXEL_GRAD_KW = (dict(), dict(Hedge=4, Wedge=6, depth_limit=3.0))
+
+
+def test_pixel_grad_sampler_bit_identical_to_reference_function(one_thread):
     """common.get_sample_uv_with_grad / get_samples_with_pixel_grad (Point-SLAM colour-gradient
     pixels, default mapping_pixels_based_on_color_grad = 1000) against the reference's own
-    functions under the same numpy seed.  skimage (absent here) is handed to the reference as
-    the scipy.ndimage restatement the mirror uses -- "parity unpinned" at rgb2gray / sobel; the
+    functions under the same numpy seed.  skimage is handed to the reference as the
+    scipy.ndimage restatement the mirror uses -- "parity unpinned" at rgb2gray / sobel; the
     selection logic (argpartition top ratio*n, region mask, np.random.choice, depth filter, ray
     construction) is the reference's own code."""
-    from types import SimpleNamespace
-    from scipy import ndimage
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip('needs /root/reference')
-    ref_harness.install()
-    import slam.common.common as rc
-    from slam.common.camera import Camera as RCam
     import xrdslam_b200.common as mc
     from xrdslam_b200.synthetic import make_sequence
-    hs = np.array([[1, 2, 1], [0, 0, 0], [-1, -2, -1]], dtype=np.float64) / 4.0
-    rc.rgb2gray = mc.rgb2gray_np
-    rc.filters = SimpleNamespace(sobel_h=lambda im: ndimage.convolve(im, hs, mode='reflect'),
-                                 sobel_v=lambda im: ndimage.convolve(im, hs.T, mode='reflect'))
+    g = load_golden_json('reference_cpu.json')['pixel_grad']
     cam, poses, fr = make_sequence(1, width=160, height=120)
-    rcam = RCam(cam.fx, cam.fy, cam.cx, cam.cy, cam.width, cam.height)
     c2w = torch.from_numpy(poses[0])
     rgb, depth = fr[0]
     np.random.seed(3)
-    a = rc.get_sample_uv_with_grad(5, 115, 7, 150, 40, rgb)
-    np.random.seed(3)
     b = mc.get_sample_uv_with_grad(5, 115, 7, 150, 40, rgb)
-    assert np.array_equal(a, b) and len(set(a.tolist())) == 40
-    for kw in (dict(), dict(Hedge=4, Wedge=6, depth_limit=3.0)):
-        np.random.seed(11)
-        ra = rc.get_samples_with_pixel_grad(rcam, 60, c2w, depth, rgb, device='cpu', **kw)
+    assert digest(b) == g['uv'] and len(set(b.tolist())) == 40
+    for kw, ref in zip(PIXEL_GRAD_KW, g['samples']):
         np.random.seed(11)
         rb = mc.get_samples_with_pixel_grad(cam, 60, c2w, depth, rgb, device='cpu', **kw)
-        assert len(ra) == len(rb) == 6
-        for x, y in zip(ra, rb):
-            assert x.dtype == y.dtype and torch.equal(x, y), kw
+        assert len(rb) == 6
+        assert [digest(y) for y in rb] == ref, kw
 
 
 def test_convonet2_load_pretrain(tmp_path):

@@ -1,51 +1,39 @@
 """CPU tests for the Vox-Fusion map structure: this package's octree (csrc/octree.cpp) against
-the reference's own svo.Octree compiled from its sources (oracle/_ref/svo.so)."""
-import os
-
+the reference's own svo.Octree compiled from its sources, through the digests stored in
+tests/golden/reference_cpu.json (tests/golden/make_golden.py reference_cpu)."""
 import numpy as np
-import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SVO = os.path.join(ROOT, 'oracle', '_ref', 'svo.so')
+from helpers import GOLDEN, digest, load_golden_json
 
 
-def ref_octree():
-    if not os.path.exists(SVO):
-        pytest.skip('oracle/_ref/svo.so not built (python oracle/build_ref.py)')
-    torch.classes.load_library(SVO)
-    o = torch.classes.svo.Octree()
-    o.init(256, 16, 0.2)
-    return o
+def octree_inserts():
+    g = torch.Generator().manual_seed(4)
+    for it in range(4):
+        pts = (torch.rand(2500, 3, generator=g) * 25 + 30 + 7 * it).int().contiguous()
+        if it == 0:
+            pts[0] = torch.tensor([0, 0, 0])
+            pts[1] = torch.tensor([254, 254, 254])
+            pts[2] = pts[3]  # duplicates
+        yield pts
 
 
 def test_octree_bit_exact_vs_reference_svo():
+    """Centres, children and features after every insert equal the reference svo.Octree's
+    (the first tree of its process, so the node ids coincide), bit for bit."""
     from xrdslam_b200 import _cabi
     lib = _cabi.lib()
-    ref = ref_octree()
-    # the reference numbers nodes with a process-global counter: offset of this tree's root
-    v0, _, _ = ref.get_centres_and_children()
+    ref = load_golden_json('reference_cpu.json')['octree']
     t = lib.xrd_octree_create(256)
-    g = torch.Generator().manual_seed(4)
     try:
-        for it in range(4):
-            pts = (torch.rand(2500, 3, generator=g) * 25 + 30 + 7 * it).int().contiguous()
-            if it == 0:
-                pts[0] = torch.tensor([0, 0, 0])
-                pts[1] = torch.tensor([254, 254, 254])
-                pts[2] = pts[3]  # duplicates
-            ref.insert(pts)
+        for pts, want in zip(octree_inserts(), ref):
             n = lib.xrd_octree_insert(t, pts.data_ptr(), pts.shape[0])
-            v, c, f = ref.get_centres_and_children()
-            assert n == v.shape[0] == lib.xrd_octree_num_nodes(t)
+            assert n == lib.xrd_octree_num_nodes(t)
             mv = torch.empty(n, 4)
             mc = torch.empty(n, 8)
             mf = torch.empty(n, 8, dtype=torch.int32)
             assert lib.xrd_octree_export(t, mv.data_ptr(), mc.data_ptr(), mf.data_ptr()) == n
-            if int(v0.shape[0]) == 1:  # first tree of the process: ids coincide
-                assert torch.equal(v, mv) and torch.equal(c, mc) and torch.equal(f, mf)
-            else:
-                assert torch.equal(v, mv)
+            assert [digest(mv), digest(mc), digest(mf)] == want
     finally:
         lib.xrd_octree_destroy(t)
 
@@ -69,28 +57,19 @@ def test_model_map_states_match_reference_formulas():
     assert int(ms['voxel_vertex_idx'].max()) < m.config.num_embeddings
 
 
-def test_vox_oracle_torch_part_matches_reference_python():
-    """oracle/voxfusion.py's features / decoder / sdf2weights / losses against the reference's
-    own SparseVoxel.render_rays + get_loss_dict run on CPU (its two CUDA ops replaced by the
-    oracle's intersections and samples, which the GPU tests pin bit-for-bit against the
-    reference's compiled kernels)."""
-    import sys
-    sys.path.insert(0, ROOT)
-    from oracle import ref_harness
-    if not ref_harness.available():
-        pytest.skip('needs /root/reference')
+def vox_case():
+    """A wall of voxels at z ~ 12.0 m (offset world), rays from above, marched by the oracle.
+    The map comes from this package's octree (bit-exact vs the reference's svo above)."""
     from oracle.voxfusion import VoxOracle
     from xrdslam_b200.camera import Camera
     from xrdslam_b200.sparse_voxel import SparseVoxelConfig
     g = torch.Generator().manual_seed(3)
-    # a wall of voxels at z ~ 12.0 m (offset world), rays from above.  The map comes from this
-    # package's octree (bit-exact vs the reference's svo above, with per-tree node ids: the
-    # reference's ids are offset by a process-global counter)
     xy = torch.rand(3000, 2, generator=g) * 2.0 + 11.0
     pts = torch.cat([xy, torch.full((3000, 1), 12.05) + torch.rand(3000, 1, generator=g) * 0.3], 1)
     builder = SparseVoxelConfig().setup(camera=Camera(320, 320, 319.5, 239.5, 640, 480))
     builder.insert_points(pts)
     voxels, children, features = builder.export_octree()
+    torch.manual_seed(5)  # the decoder keeps torch's default init
     ora = VoxOracle(seed=5)
     ora.set_map(voxels, children, features)
     with torch.no_grad():
@@ -107,38 +86,40 @@ def test_vox_oracle_torch_part_matches_reference_python():
     td = torch.full((R, 1), 1.62) + torch.rand(R, 1, generator=g) * 0.2
     td[5::11] = 0
     ts = torch.rand(R, 3, generator=g)
-    # the reference model on the same map / decoder / embeddings
     ms = {'voxel_vertex_idx': ora.vertex_idx, 'voxel_center_xyz': ora.centres,
           'voxel_structure': ora.children}
     full_inter = {k: torch.zeros((R,) + v.shape[1:], dtype=v.dtype) for k, v in inter.items()}
     for k in full_inter:
         full_inter[k][hits] = inter[k]
-    ref, sv = ref_harness.ref_sparse_voxel_cpu(ms, ora.embeddings.detach(), (full_inter, hits, samples))
-    rsd = ref.decoder.state_dict()
-    with torch.no_grad():
-        od = ora.decoder
-        od.pts_linears[0].weight.copy_(rsd['pts_linears.0.weight']); od.pts_linears[0].bias.copy_(rsd['pts_linears.0.bias'])
-        od.pts_linears[1].weight.copy_(rsd['pts_linears.1.weight']); od.pts_linears[1].bias.copy_(rsd['pts_linears.1.bias'])
-        od.sdf_out.weight.copy_(rsd['sdf_out.weight']); od.sdf_out.bias.copy_(rsd['sdf_out.bias'])
-        od.color_out[0].weight.copy_(rsd['color_out.0.weight']); od.color_out[0].bias.copy_(rsd['color_out.0.bias'])
-        od.color_out[2].weight.copy_(rsd['color_out.2.weight']); od.color_out[2].bias.copy_(rsd['color_out.2.bias'])
+    return ora, ro, rd, ts, td, marched, ms, full_inter
+
+
+def test_vox_oracle_torch_part_matches_reference_python(one_thread):
+    """oracle/voxfusion.py's features / decoder / sdf2weights / losses against the reference's
+    own SparseVoxel.render_rays + get_loss_dict run on CPU on the same map, decoder, embeddings,
+    intersections and samples (its two CUDA ops replaced by the oracle's intersections and
+    samples, which the GPU tests pin bit-for-bit against the reference's compiled kernels)."""
+    import os
+    g = load_golden_json('reference_cpu.json')['vox']
+    a = np.load(os.path.join(GOLDEN, 'reference_cpu.npz'))
+    r = lambda k: torch.from_numpy(a['vox.' + k])
+    ora, ro, rd, ts, td, marched, _, _ = vox_case()
+    od = ora.decoder
     out_o, ld_o = ora.render(ro, rd, ts, td, marched)
-    with ref_harness.cuda_calls_are_noops():
-        out_r = ref.render_rays(ro.unsqueeze(0), rd.unsqueeze(0), target_d=td.unsqueeze(0))
-    ld_r = ref.get_loss_dict(out_r, {'target_d': td, 'target_s': ts}, True)
-    assert torch.equal(out_r['ray_mask'], out_o['ray_mask'])
-    assert (out_r['depth'] - out_o['depth']).abs().max() < 1e-6
-    assert (out_r['rgb'] - out_o['rgb']).abs().max() < 1e-6
-    assert (out_r['sdf'] - out_o['sdf']).abs().max() < 1e-6
-    for k in ld_r:
-        assert abs(float(ld_r[k]) - float(ld_o[k])) <= 1e-5 * max(1e-3, abs(float(ld_r[k]))), k
+    assert digest(out_o['ray_mask']) == g['ray_mask']
+    assert (r('depth') - out_o['depth']).abs().max() < 1e-6
+    assert (r('rgb') - out_o['rgb']).abs().max() < 1e-6
+    assert (r('sdf') - out_o['sdf']).abs().max() < 1e-6
+    assert set(ld_o) == set(g['losses'])
+    for k, v in g['losses'].items():
+        assert abs(v - float(ld_o[k].detach())) <= 1e-5 * max(1e-3, abs(v)), k
     # gradients of the summed loss w.r.t. embeddings and decoder
     sum(ld_o.values()).backward()
-    sum(ld_r.values()).backward()
-    ge_o, ge_r = ora.embeddings.grad, ref.embeddings.grad
-    assert (ge_o - ge_r).abs().max() <= 1e-5 * ge_r.abs().max()
-    assert (od.sdf_out.weight.grad - ref.decoder.sdf_out.weight.grad).abs().max() <= \
-        1e-5 * ref.decoder.sdf_out.weight.grad.abs().max()
+    ge_r = torch.zeros_like(ora.embeddings)
+    ge_r[r('d_embeddings_rows')] = r('d_embeddings')
+    assert (ora.embeddings.grad - ge_r).abs().max() <= 1e-5 * ge_r.abs().max()
+    assert (od.sdf_out.weight.grad - r('d_sdf_out_w')).abs().max() <= \
+        1e-5 * r('d_sdf_out_w').abs().max()
 
 
 def test_device_octree_equals_host_octree_numbering():

@@ -1,30 +1,76 @@
 """Vox-Fusion GPU parity: (1) the raw intersection / sampling kernels bit-for-bit against the
-reference's OWN `grid` CUDA extension (compiled from the reference sources into
-oracle/_ref/grid.so), (2) the full march + render step against oracle/voxfusion.py."""
-import importlib.machinery
-import importlib.util
-import os
+reference's OWN `grid` CUDA extension, (2) the full march + render step against
+oracle/voxfusion.py.  The reference extension's outputs on these seeded scenes are stored as
+SHA-256 digests in tests/golden/vox_grid_ref.json (tests/golden/make_golden.py vox_grid runs
+the extension, compiled from the reference sources by oracle/build_ref.py, on a B200)."""
+import ctypes as C
 
 import numpy as np
 import pytest
 import torch
 
-from helpers import max_abs, rel_err
+from helpers import digest, load_golden_json, max_abs, rel_err
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-GRID = os.path.join(ROOT, 'oracle', '_ref', 'grid.so')
 OFFSET = 25.6  # voxels_each_dim / 2 * voxel_size: keeps coordinates inside [0, 256) voxels
 
 
-def ref_grid():
-    if not os.path.exists(GRID):
-        pytest.skip('oracle/_ref/grid.so not built')
-    loader = importlib.machinery.ExtensionFileLoader('grid', GRID)
-    spec = importlib.util.spec_from_loader('grid', loader)
-    mod = importlib.util.module_from_spec(spec)
-    loader.exec_module(mod)
-    return mod
+def golden():
+    return load_golden_json('vox_grid_ref.json')
+
+
+class OwnGrid:
+    """This package's raw intersection / sampling kernels behind the call signatures of the
+    reference's `grid` extension (svo_intersect, inverse_cdf_sampling)."""
+
+    def __init__(self, dev):
+        from xrdslam_b200 import _cabi
+        self.dev, self.cabi, self.lib = dev, _cabi, _cabi.lib()
+
+    def svo_intersect(self, ro, rd, cen, ch, vs, n_max):
+        ro, rd = ro[0].float().contiguous(), rd[0].float().contiguous()
+        cen, ch = cen[0].float().contiguous(), ch[0].int().contiguous()
+        R = ro.shape[0]
+        idx = torch.empty(R, n_max, dtype=torch.int32, device=self.dev)
+        lo = torch.empty(R, n_max, device=self.dev)
+        hi = torch.empty(R, n_max, device=self.dev)
+        rays = self.cabi.XrdRays(R, ro.data_ptr(), rd.data_ptr(), None, None)
+        mp = self.cabi.XrdVoxMap(cen.shape[0], cen.data_ptr(), ch.data_ptr(), None, None, 0)
+        self.cabi.check('xrd_voxfusion_intersect_raw', self.lib.xrd_voxfusion_intersect_raw(
+            C.byref(rays), C.byref(mp), vs, n_max, idx.data_ptr(), lo.data_ptr(), hi.data_ptr(),
+            None))
+        return idx[None], lo[None], hi[None]
+
+    def inverse_cdf_sampling(self, pi, mn, mx, noise, pr, stp, fixed):
+        G, K, P = pi.shape
+        ms = noise.shape[-1]
+        s_idx = torch.empty(G * K, ms, dtype=torch.int32, device=self.dev)
+        s_depth = torch.empty(G * K, ms, device=self.dev)
+        s_dist = torch.empty(G * K, ms, device=self.dev)
+        c = lambda t: t.contiguous().data_ptr()
+        self.cabi.check('xrd_voxfusion_sample_raw', self.lib.xrd_voxfusion_sample_raw(
+            G * K, P, ms, K, c(pi), c(mn), c(mx), c(noise), c(pr), c(stp), s_idx.data_ptr(),
+            s_depth.data_ptr(), s_dist.data_ptr(), None))
+        return s_idx.reshape(G, K, ms), s_depth.reshape(G, K, ms), s_dist.reshape(G, K, ms)
+
+
+class Recorder:
+    """Wraps a `grid` implementation and keeps the digests of every output it returns, in call
+    order (intersection t values only where a voxel was hit)."""
+
+    def __init__(self, grid):
+        self.grid, self.digests = grid, []
+
+    def svo_intersect(self, *a):
+        idx, lo, hi = self.grid.svo_intersect(*a)
+        m = idx >= 0
+        self.digests += [digest(idx), digest(lo[m]), digest(hi[m])]
+        return idx, lo, hi
+
+    def inverse_cdf_sampling(self, *a):
+        out = self.grid.inverse_cdf_sampling(*a)
+        self.digests += [digest(t) for t in out]
+        return out
 
 
 def scene(device, n_frames=2, R=700, seed=0):
@@ -57,40 +103,23 @@ def scene(device, n_frames=2, R=700, seed=0):
     return model, rays_o, rays_d, ts, td
 
 
-def test_intersect_kernel_bit_exact_vs_reference_grid(cuda_dev):
-    import ctypes as C
-    from xrdslam_b200 import _cabi
-    grid = ref_grid()
-    model, rays_o, rays_d, _, _ = scene(cuda_dev)
+def intersect_case(grid, dev):
+    """The reference call exactly as voxel_helpers_voxfusion.py:237-255 would issue it with
+    G = 1, on the map and rays of scene(dev)."""
+    model, rays_o, rays_d, _, _ = scene(dev)
     ms = model.map_states
-    ro, rd = rays_o.to(cuda_dev), rays_d.to(cuda_dev)
-    R = ro.shape[0]
-    # reference call exactly as voxel_helpers_voxfusion.py:237-255 would issue it with G = 1
-    inds, tmin, tmax = grid.svo_intersect(ro[None].contiguous(), rd[None].contiguous(),
-                                          ms['voxel_center_xyz'][None].contiguous(),
-                                          ms['voxel_structure'][None].contiguous(), 0.2, 50)
-    idx = torch.empty(R, 50, dtype=torch.int32, device=cuda_dev)
-    lo = torch.empty(R, 50, device=cuda_dev)
-    hi = torch.empty(R, 50, device=cuda_dev)
-    rays = _cabi.XrdRays(R, ro.data_ptr(), rd.data_ptr(), None, None)
-    mp = model._map_struct(model.embeddings.detach())
-    st = _cabi.lib().xrd_voxfusion_intersect_raw(C.byref(rays), C.byref(mp), 0.2, 50,
-                                                 idx.data_ptr(), lo.data_ptr(), hi.data_ptr(), None)
-    _cabi.check('xrd_voxfusion_intersect_raw', st)
-    torch.cuda.synchronize()
-    assert torch.equal(idx, inds[0])  # node ids, visiting order: bit-exact
-    m = idx >= 0
-    assert m.sum() > R  # plenty of hits
-    assert torch.equal(lo[m], tmin[0][m]) and torch.equal(hi[m], tmax[0][m])  # t values bit-exact
+    ro, rd = rays_o.to(dev), rays_d.to(dev)
+    return grid.svo_intersect(ro[None].contiguous(), rd[None].contiguous(),
+                              ms['voxel_center_xyz'][None].contiguous(),
+                              ms['voxel_structure'][None].contiguous(), 0.2, 50)
 
 
-def test_sampling_kernel_bit_exact_vs_reference_grid(cuda_dev):
+def sampling_case(grid, dev):
+    """Intersections through `grid`, then the inputs of ray_sample + InverseCDFRaySampling.forward
+    (voxel_helpers_voxfusion.py:399-481,690-714) for scene(dev, R=900)."""
     from oracle.voxfusion import ray_intersect
-    from xrdslam_b200 import _cabi
-    grid = ref_grid()
-    model, rays_o, rays_d, _, _ = scene(cuda_dev, R=900)
+    model, rays_o, rays_d, _, _ = scene(dev, R=900)
     ms = model.map_states
-    dev = cuda_dev
 
     def gpu_intersect(ro, rd, cen, ch, vs, n_max):
         i, a, b = grid.svo_intersect(ro[None].to(dev).contiguous(), rd[None].to(dev).contiguous(),
@@ -99,7 +128,6 @@ def test_sampling_kernel_bit_exact_vs_reference_grid(cuda_dev):
     inter, hits = ray_intersect(rays_o, rays_d, ms['voxel_center_xyz'], ms['voxel_structure'],
                                 0.2, intersect_fn=gpu_intersect)
     inter = {k: v[hits].to(dev) for k, v in inter.items()}
-    # ray_sample + InverseCDFRaySampling.forward (voxel_helpers_voxfusion.py:399-481,690-714)
     dists = (inter['max_depth'] - inter['min_depth']).masked_fill(
         inter['intersected_voxel_idx'].eq(-1), 0)
     probs = dists / dists.sum(dim=-1, keepdim=True)
@@ -113,23 +141,30 @@ def test_sampling_kernel_bit_exact_vs_reference_grid(cuda_dev):
     max_steps = int(steps.ceil().long().max()) + P
     gen = torch.Generator(device='cpu').manual_seed(3)
     noise = torch.rand(G, K, max_steps, generator=gen).clamp(min=0.001, max=0.999).to(dev)
-    r_idx, r_depth, r_dist = grid.inverse_cdf_sampling(
-        pi.reshape(G, K, P).contiguous(), mn.reshape(G, K, P).contiguous(),
-        mx.reshape(G, K, P).contiguous(), noise.contiguous(), pr.reshape(G, K, P).contiguous(),
-        stp.reshape(G, K).contiguous(), -1)
-    s_idx = torch.empty(Hh, max_steps, dtype=torch.int32, device=dev)
-    s_depth = torch.empty(Hh, max_steps, device=dev)
-    s_dist = torch.empty(Hh, max_steps, device=dev)
-    st = _cabi.lib().xrd_voxfusion_sample_raw(
-        Hh, P, max_steps, K, pi.contiguous().data_ptr(), mn.contiguous().data_ptr(),
-        mx.contiguous().data_ptr(), noise.reshape(Hh, max_steps).data_ptr(),
-        pr.contiguous().data_ptr(), stp.contiguous().data_ptr(), s_idx.data_ptr(),
-        s_depth.data_ptr(), s_dist.data_ptr(), None)
-    _cabi.check('xrd_voxfusion_sample_raw', st)
-    torch.cuda.synchronize()
-    assert torch.equal(s_idx, r_idx.reshape(Hh, -1))      # voxel of every sample: bit-exact
-    assert torch.equal(s_depth, r_depth.reshape(Hh, -1))  # mid-point depths: bit-exact
-    assert torch.equal(s_dist, r_dist.reshape(Hh, -1))
+    return (pi.reshape(G, K, P).contiguous(), mn.reshape(G, K, P).contiguous(),
+            mx.reshape(G, K, P).contiguous(), noise.contiguous(), pr.reshape(G, K, P).contiguous(),
+            stp.reshape(G, K).contiguous(), -1)
+
+
+def test_intersect_kernel_bit_exact_vs_reference_grid(cuda_dev):
+    """Node ids in visiting order and the t values of every hit equal the reference
+    extension's, bit for bit."""
+    rec = Recorder(OwnGrid(cuda_dev))
+    idx, _, _ = intersect_case(rec, cuda_dev)
+    assert (idx >= 0).sum() > idx.shape[1]  # plenty of hits
+    assert rec.digests == golden()['intersect']
+
+
+def test_sampling_kernel_bit_exact_vs_reference_grid(cuda_dev):
+    """Voxel, mid-point depth and distance of every sample equal the reference extension's,
+    bit for bit, on the same intersections (themselves checked against the reference's)."""
+    rec = Recorder(OwnGrid(cuda_dev))
+    args = sampling_case(rec, cuda_dev)
+    g = golden()['sampling']
+    assert rec.digests == g['intersect']
+    rec.digests = []
+    rec.inverse_cdf_sampling(*args)
+    assert rec.digests == g['samples']
 
 
 @pytest.mark.parametrize('need_pose', [True, False])
@@ -207,12 +242,12 @@ def test_no_hit_returns_none(cuda_dev):
     assert out is None  # reference: render_rays prints "no hit" and returns None
 
 
-def _march_through_reference_grid(grid, ora, rays_o, rays_d, noise_fn, dev):
-    """VoxOracle.march with BOTH native stages executed by the reference's own compiled CUDA
-    extension (oracle/_ref/grid.so: svo_intersect + inverse_cdf_sampling), glued exactly as
-    voxel_helpers_voxfusion.py:237-255,399-481 glue them.  The CPU restatement divides
-    exactly where the reference kernels use __fdividef; chained through grid.so the oracle
-    sees the reference's own bits (VERDICT r01 weak item 4)."""
+def _march_through_grid(grid, ora, rays_o, rays_d, noise_fn, dev):
+    """VoxOracle.march with BOTH native stages executed by `grid` (svo_intersect +
+    inverse_cdf_sampling), glued exactly as voxel_helpers_voxfusion.py:237-255,399-481 glue
+    them.  The CPU restatement divides exactly where the reference kernels use __fdividef;
+    chained through bits equal to the reference extension's, the oracle sees the reference's
+    own bits."""
     from oracle.voxfusion import MAX_DEPTH, ray_intersect
 
     def gpu_intersect(ro, rd, cen, ch, vs, n_max):
@@ -252,16 +287,11 @@ def _march_through_reference_grid(grid, ora, rays_o, rays_d, noise_fn, dev):
     return inter, hits, samples
 
 
-@pytest.mark.parametrize('R', [300, 5 * 1024])
-def test_full_step_vs_oracle_chained_through_reference_grid(cuda_dev, R):
-    """Full step (march + sample + decode + composite + loss + backward) with the oracle fed
-    the reference extension's own intersections / samples: sample->voxel ids and depths
-    BIT-EXACT, gradients rel-l2 <= 5e-4.  R = 5 x 1024 is the default mapping batch
-    (5 keyframes x 1024 rays, slam/configs/input_config.py vox-fusion entry)."""
+def chained_case(dev, R):
+    """Model and oracle on the same map, embeddings and decoder, with the noise drawn by hit
+    rank, for the chained full-step test."""
     from oracle.voxfusion import VoxOracle
-    grid = ref_grid()
-    model, rays_o, rays_d, ts, td = scene(cuda_dev, R=R, seed=4)
-    dev = cuda_dev
+    model, rays_o, rays_d, ts, td = scene(dev, R=R, seed=4)
     ora = VoxOracle()
     with torch.no_grad():
         g = torch.Generator().manual_seed(9)
@@ -280,9 +310,23 @@ def test_full_step_vs_oracle_chained_through_reference_grid(cuda_dev, R):
         n = min(G * K, noise_rank.shape[0])
         out[:n] = noise_rank[:n, :ms]
         return out.reshape(G, K, ms)
+    return model, ora, rays_o, rays_d, ts, td, noise_rank, noise_fn
+
+
+@pytest.mark.parametrize('R', [300, 5 * 1024])
+def test_full_step_vs_oracle_chained_through_reference_grid(cuda_dev, R):
+    """Full step (march + sample + decode + composite + loss + backward) with the oracle fed
+    intersections / samples bit-identical to the reference extension's own (every one checked
+    against its stored digest): sample->voxel ids and depths BIT-EXACT, gradients rel-l2
+    <= 5e-4.  R = 5 x 1024 is the default mapping batch (5 keyframes x 1024 rays,
+    slam/configs/input_config.py vox-fusion entry)."""
+    dev = cuda_dev
+    model, ora, rays_o, rays_d, ts, td, noise_rank, noise_fn = chained_case(dev, R)
+    grid = Recorder(OwnGrid(dev))
     ro_o = rays_o.clone().requires_grad_(True)
     rd_o = rays_d.clone().requires_grad_(True)
-    marched = _march_through_reference_grid(grid, ora, ro_o.detach(), rd_o.detach(), noise_fn, dev)
+    marched = _march_through_grid(grid, ora, ro_o.detach(), rd_o.detach(), noise_fn, dev)
+    assert grid.digests == golden()['chained'][str(R)]
     out_o, ld_o = ora.render(ro_o, rd_o, ts, td, marched)
     sum(ld_o.values()).backward()
     hits = marched[1]
