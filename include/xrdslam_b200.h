@@ -540,10 +540,55 @@ typedef struct {
 
 size_t xrd_voxfusion_render_workspace_bytes(int n_rays, int n_points, int with_grads);
 
+/* Point query of the mesher path (slam/model_components/voxel_helpers_voxfusion.py:15-95
+ * get_scores / eval_points): trilinear embedding of the voxel's 8 vertex embeddings
+ * (get_features :106-153) and the decoder forward (decoder_voxfusion.py:122-140 get_values) at
+ * DEVICE points [P,3] fp32, each with its voxel id (DEVICE [P] int32, a row of map->centres /
+ * map->vertex_idx).  raw: DEVICE [P,4] = (rgb after the colour head's sigmoid, sdf).  The
+ * workspace is forward-only. */
+size_t xrd_voxfusion_query_workspace_bytes(int n_points);
+int xrd_voxfusion_query(const XrdVoxMap* map, const XrdVoxDecoder* dec, float voxel_size,
+                        const float* points, const int32_t* voxel_ids, int n_points, float* raw,
+                        void* workspace, size_t workspace_bytes, void* stream);
+
 int xrd_voxfusion_render(const XrdRays* rays, const XrdVoxMap* map, const XrdVoxMarch* march,
                          const XrdVoxMarchCfg* mcfg, const XrdVoxDecoder* dec,
                          const XrdVoxRenderCfg* cfg, XrdVoxOut* out, XrdVoxGrads* grads,
                          void* workspace, size_t workspace_bytes, void* stream);
+
+/* ---- Marching cubes -----------------------------------------------------------
+ *
+ *   xrd_mc_count / xrd_mc_emit  the isosurface step of the mesher: skimage.measure.marching_cubes
+ *                               on the host in slam/common/mesher.py:203-233 (one 256^3 volume)
+ *                               and slam/algorithms/voxfusion.py:253-279 (one call per voxel).
+ * A batch of B fp32 volumes [B][nx][ny][nz] (x slowest).  A corner is inside when value < level;
+ * a lattice edge whose ends lie on opposite sides gets one vertex (welded inside a volume, never
+ * across volumes) at
+ *   t = (level - v0) / (v1 - v0)                        fp32, v0 = lower-index end
+ *   world_d = origin_d + (i_d + t * e_d) * spacing_d    fp64, stored as fp32.
+ * Vertices are ordered by (volume, i, j, k, axis), faces by (volume, cube, table order); the
+ * output is bit-identical run to run.  Winding: the right-hand normal of every triangle points
+ * toward increasing field values.  Case tables and the ambiguous-face rule:
+ * scripts/gen_mc_tables.py.
+ *
+ * xrd_mc_count writes (V, F) to DEVICE counts[2]; the caller reads them, allocates
+ * verts [V,3] fp32 and faces [F,3] int32 and calls xrd_mc_emit with the same volumes, level and
+ * the UNTOUCHED workspace (it holds the scans between the two calls). */
+typedef struct {
+  const float* field;      /* DEVICE [n_volumes][nx][ny][nz]                                   */
+  int n_volumes, nx, ny, nz; /* nx, ny, nz >= 2                                               */
+  double origin[3];        /* world position of lattice point (0,0,0), shared by all volumes   */
+  double spacing[3];       /* lattice step per axis, shared                                    */
+  const double* origins;   /* DEVICE [n_volumes][3] per-volume origin, or NULL: origin[]       */
+  const double* spacings;  /* DEVICE [n_volumes][3] per-volume spacing, or NULL: spacing[]     */
+} XrdMcVolumes;
+
+size_t xrd_mc_workspace_bytes(int n_volumes, int nx, int ny, int nz);
+int xrd_mc_count(const XrdMcVolumes* v, float level, int* counts, void* workspace,
+                 size_t workspace_bytes, void* stream);
+/* verts or faces may be NULL (skipped). */
+int xrd_mc_emit(const XrdMcVolumes* v, float level, float* verts, int32_t* faces, void* workspace,
+                size_t workspace_bytes, void* stream);
 
 /* ---- Point-SLAM -------------------------------------------------------------
  *

@@ -165,6 +165,12 @@ class XrdVoxGrads(C.Structure):
                 ('d_rays_o', vp), ('d_rays_d', vp)]
 
 
+class XrdMcVolumes(C.Structure):
+    _fields_ = [('field', vp), ('n_volumes', C.c_int), ('nx', C.c_int), ('ny', C.c_int),
+                ('nz', C.c_int), ('origin', C.c_double * 3), ('spacing', C.c_double * 3),
+                ('origins', vp), ('spacings', vp)]
+
+
 class XrdPointIndex(C.Structure):
     _fields_ = [('pos', vp), ('n_points', C.c_int), ('cell', C.c_float),
                 ('table_size', C.c_int), ('cell_start', vp), ('cell_end', vp),
@@ -274,6 +280,12 @@ SYMBOLS = {
         C.POINTER(XrdRays), C.POINTER(XrdVoxMap), C.POINTER(XrdVoxMarch),
         C.POINTER(XrdVoxMarchCfg), C.POINTER(XrdVoxDecoder), C.POINTER(XrdVoxRenderCfg),
         C.POINTER(XrdVoxOut), C.POINTER(XrdVoxGrads), vp, C.c_size_t, vp]),
+    'xrd_voxfusion_query_workspace_bytes': (C.c_size_t, [C.c_int]),
+    'xrd_voxfusion_query': (C.c_int, [C.POINTER(XrdVoxMap), C.POINTER(XrdVoxDecoder), C.c_float,
+                                      vp, vp, C.c_int, vp, vp, C.c_size_t, vp]),
+    'xrd_mc_workspace_bytes': (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
+    'xrd_mc_count': (C.c_int, [C.POINTER(XrdMcVolumes), C.c_float, vp, vp, C.c_size_t, vp]),
+    'xrd_mc_emit': (C.c_int, [C.POINTER(XrdMcVolumes), C.c_float, vp, vp, vp, C.c_size_t, vp]),
     'xrd_pointslam_knn_query': (C.c_int, [C.POINTER(XrdPointIndex), vp, vp, C.c_int, C.c_int,
                                           vp, vp, vp, vp]),
     'xrd_coslam_query': (C.c_int, [C.POINTER(XrdHashGrid), C.POINTER(XrdCoslamMlp), vp, C.c_int,

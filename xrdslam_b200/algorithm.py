@@ -70,6 +70,10 @@ class Algorithm():
     def render_img(self, c2w, gt_depth=None, idx=None):
         return None, None
 
+    def get_mesh(self):
+        """base_algorithm.py:89-91: algorithms without a mesher return None."""
+        return None
+
     def optimizer_config_update(self, max_iters, coarse=False):
         pass
 

@@ -14,6 +14,7 @@ import torch
 from .algorithm import Algorithm, AlgorithmConfig
 from .common import get_camera_rays, get_rays, get_samples, rays_from_poses
 from .joint_encoding import JointEncodingConfig
+from .mesher import MesherConfig
 from .opt_pose import pose_matrices
 from .optimizers import AdamOptimizerConfig, Optimizers
 
@@ -41,6 +42,7 @@ class CoSLAMConfig(AlgorithmConfig):
     _target: Type = field(default_factory=lambda: CoSLAM)
     model: JointEncodingConfig = field(default_factory=lambda: JointEncodingConfig(
         cam_depth_trunc=100.0, tcnn_encoding=True))
+    mesher: MesherConfig = field(default_factory=MesherConfig)
     separate_LR: bool = True
     retain_graph: bool = True
     rot_rep: str = 'axis_angle'
@@ -105,6 +107,9 @@ class CoSLAM(Algorithm):
         self.model = self.config.model.setup(camera=camera,
                                              bounding_box=self.bounding_box)
         self.model.to(device)
+        self.mesher = self.config.mesher.setup(camera=camera, bounding_box=self.bounding_box,
+                                               marching_cubes_bound=self.marching_cube_bound)
+        self.cur_mesh = None
         self.bundle_adjust = True
         self.num_rays_to_save = int(self.camera.width * self.camera.height *
                                     self.config.rays_to_save_ratio)
@@ -336,3 +341,12 @@ class CoSLAM(Algorithm):
             color = torch.cat(colors, 0).reshape(self.camera.height,
                                                  self.camera.width, 3)
             return color.cpu().numpy(), depth.cpu().numpy()
+
+    # coslam.py:291-298
+    def get_mesh(self):
+        with self.lock:
+            self.cur_mesh = self.mesher.get_mesh(keyframe_graph=self.keyframe_graph,
+                                                 query_fn=self.model.query_fn,
+                                                 color_func=self.model.color_func,
+                                                 device=self.device)
+            return self.cur_mesh

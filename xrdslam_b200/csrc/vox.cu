@@ -314,6 +314,8 @@ struct PointParams {
   float* d_emb;
   float* dp;          // [3][P]
   int need_dp;
+  // query mode: sample points given directly (pt_ray / pt_k unused)
+  const float* pts; const int* pts_vox;
 };
 // activation rows: h1 | h2 | feat | x   (feat and x adjacent: the colour net's 144-wide input
 // cat[feat, x] is one GEMM operand) | c1
@@ -339,13 +341,11 @@ struct Corner {
   float w[8];
   float p[3];
 };
-__device__ __forceinline__ void corners(const PointParams& P, int r, int k, float xyz[3], Corner& c) {
-  const float depth = P.smp_depth[(size_t)r * P.scap + k];
-  const int vox = P.smp_idx[(size_t)r * P.scap + k];
+// p = (xyz - centre) / voxel_size + 0.5 and the 8 trilinear weights of voxel `vox`
+__device__ __forceinline__ void corners_at(const PointParams& P, const float xyz[3], int vox,
+                                           Corner& c) {
 #pragma unroll
   for (int d = 0; d < 3; ++d) {
-    xyz[d] = __fadd_rn(P.rays_o[r * 3 + d], __fmul_rn(P.rays_d[r * 3 + d], depth));
-    // p = (xyz - centre) / voxel_size + 0.5
     c.p[d] = __fadd_rn(__fdiv_rn(__fsub_rn(xyz[d], P.centres[vox * 3 + d]), P.voxel_size), 0.5f);
   }
 #pragma unroll
@@ -358,6 +358,13 @@ __device__ __forceinline__ void corners(const PointParams& P, int r, int k, floa
     c.w[i] = wx * wy * wz;
   }
 }
+__device__ __forceinline__ void corners(const PointParams& P, int r, int k, float xyz[3], Corner& c) {
+  const float depth = P.smp_depth[(size_t)r * P.scap + k];
+#pragma unroll
+  for (int d = 0; d < 3; ++d)
+    xyz[d] = __fadd_rn(P.rays_o[r * 3 + d], __fmul_rn(P.rays_d[r * 3 + d], depth));
+  corners_at(P, xyz, P.smp_idx[(size_t)r * P.scap + k], c);
+}
 
 // ---- GEMM decoder path: gather / head / scatter kernels around gemm.cuh -------------------
 // x = trilinear embedding of the sample point -> activation rows ra_x
@@ -366,7 +373,13 @@ __global__ void __launch_bounds__(T) k_vox_gather(const PointParams P) {
   if (p >= P.P) return;
   float xyz[3];
   Corner c;
-  corners(P, P.pt_ray[p], P.pt_k[p], xyz, c);
+  if (P.pts) {  // free query points (xrd_voxfusion_query)
+#pragma unroll
+    for (int d = 0; d < 3; ++d) xyz[d] = P.pts[(size_t)p * 3 + d];
+    corners_at(P, xyz, P.pts_vox[p], c);
+  } else {
+    corners(P, P.pt_ray[p], P.pt_k[p], xyz, c);
+  }
   float x[EMB];
 #pragma unroll
   for (int q = 0; q < EMB; ++q) x[q] = 0.f;
@@ -726,6 +739,71 @@ VWs vws(int R, int Pn, int with_grads) {
 }
 }  // namespace
 
+#define XRD_GEMM(...)                                         \
+  do {                                                        \
+    GemmArgs g_ = __VA_ARGS__;                                \
+    XRD_CUDA_TRY(launch_gemm(g_, stream));                    \
+  } while (0)
+
+// Embedding gather + decoder (decoder_voxfusion.py:122-149) as GEMMs over [feature][point] rows:
+// Q.sdf [P] and Q.rgb [3][P] (after the colour head's sigmoid); activations stay in Q.acts.
+static int vox_forward(const PointParams& Q, const XrdVoxDecoder* dec, cudaStream_t stream) {
+  const int Pn = Q.P, Pp = Q.Pp;
+  auto ar = [&](int row) { return Q.acts + (size_t)row * Pp; };
+  k_vox_gather<<<(Pn + T - 1) / T, T, 0, stream>>>(Q);
+  XRD_LAUNCH_CHECK();
+  XRD_GEMM({W, Pn, EMB, dec->w0, EMB, 0, ar(ra_x()), Pp, ar(ra_h1()), Pp, dec->b0, ACT_RELU});
+  XRD_GEMM({W, Pn, W, dec->w1, W, 0, ar(ra_h1()), Pp, ar(ra_h2()), Pp, dec->b1, ACT_RELU});
+  // sdf_out: torch row 0 = sdf, rows 1..128 = feat
+  XRD_GEMM({W, Pn, W, dec->ws + W, W, 0, ar(ra_h2()), Pp, ar(ra_feat()), Pp, dec->bs + 1, ACT_NONE});
+  XRD_GEMM({1, Pn, W, dec->ws, W, 0, ar(ra_h2()), Pp, Q.sdf, Pn, dec->bs, ACT_NONE});
+  // colour: relu(wc0 [feat, x] + bc0) -> sigmoid(wc1 . + bc1)
+  XRD_GEMM({W, Pn, W + EMB, dec->wc0, W + EMB, 0, ar(ra_feat()), Pp, ar(ra_c1()), Pp, dec->bc0, ACT_RELU});
+  XRD_GEMM({3, Pn, W, dec->wc1, W, 0, ar(ra_c1()), Pp, Q.rgb, Pn, dec->bc1, ACT_SIGMOID});
+  return XRD_OK;
+}
+
+__global__ void __launch_bounds__(256) k_vox_pack_raw(int P, const float* rgb, const float* sdf,
+                                                      float* raw) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= P) return;
+  raw[(size_t)p * 4 + 0] = rgb[p];
+  raw[(size_t)p * 4 + 1] = rgb[(size_t)P + p];
+  raw[(size_t)p * 4 + 2] = rgb[(size_t)2 * P + p];
+  raw[(size_t)p * 4 + 3] = sdf[p];
+}
+
+extern "C" size_t xrd_voxfusion_query_workspace_bytes(int n_points) {
+  return vws(0, n_points, 0).total;
+}
+
+extern "C" int xrd_voxfusion_query(const XrdVoxMap* map, const XrdVoxDecoder* dec, float voxel_size,
+                                   const float* points, const int32_t* voxel_ids, int n_points,
+                                   float* raw, void* workspace, size_t workspace_bytes,
+                                   void* stream_) {
+  if (!map || !dec || !workspace) return XRD_E_NULL;
+  if (n_points < 0) return XRD_E_SHAPE;
+  if (n_points == 0) return XRD_OK;
+  if (!points || !voxel_ids || !raw || !map->centres || !map->vertex_idx || !map->embeddings)
+    return XRD_E_NULL;
+  const VWs L = vws(0, n_points, 0);
+  if (workspace_bytes < L.total) return XRD_E_WORKSPACE;
+  cudaStream_t stream = (cudaStream_t)stream_;
+  char* ws = reinterpret_cast<char*>(workspace);
+  PointParams Q{};
+  Q.P = n_points; Q.Pp = (int)align_up((size_t)n_points, 64);
+  Q.pts = points; Q.pts_vox = voxel_ids;
+  Q.centres = map->centres; Q.vertex_idx = map->vertex_idx; Q.emb = map->embeddings;
+  Q.voxel_size = voxel_size; Q.dec = *dec;
+  Q.acts = reinterpret_cast<float*>(ws + L.acts);
+  Q.sdf = reinterpret_cast<float*>(ws + L.sdf); Q.rgb = reinterpret_cast<float*>(ws + L.rgb);
+  const int st = vox_forward(Q, dec, stream);
+  if (st != XRD_OK) return st;
+  k_vox_pack_raw<<<(n_points + 255) / 256, 256, 0, stream>>>(n_points, Q.rgb, Q.sdf, raw);
+  XRD_LAUNCH_CHECK();
+  return XRD_OK;
+}
+
 extern "C" size_t xrd_voxfusion_render_workspace_bytes(int n_rays, int n_points, int with_grads) {
   return vws(n_rays, n_points, with_grads).total;
 }
@@ -764,26 +842,13 @@ extern "C" int xrd_voxfusion_render(const XrdRays* rays, const XrdVoxMap* map,
   Q.sdf = reinterpret_cast<float*>(ws + L.sdf); Q.rgb = reinterpret_cast<float*>(ws + L.rgb);
   Q.d_sdf = nullptr; Q.d_rgb = nullptr; Q.grads = nullptr; Q.d_emb = nullptr; Q.dp = nullptr;
   Q.need_dp = 0;
-  // decoder (decoder_voxfusion.py:122-149) as GEMMs over [feature][point] rows
+  Q.pts = nullptr; Q.pts_vox = nullptr;
   auto ar = [&](int row) { return Q.acts + (size_t)row * Pp; };
-#define XRD_GEMM(...)                                         \
-  do {                                                        \
-    GemmArgs g_ = __VA_ARGS__;                                \
-    XRD_CUDA_TRY(launch_gemm(g_, stream));                    \
-  } while (0)
   {
   // timed bracket = the forward decoder chain: gather + 6 GEMM launches (bench.py's roofline)
   KernelTimer kt(stream);
-  k_vox_gather<<<(Pn + T - 1) / T, T, 0, stream>>>(Q);
-  XRD_LAUNCH_CHECK();
-  XRD_GEMM({W, Pn, EMB, dec->w0, EMB, 0, ar(ra_x()), Pp, ar(ra_h1()), Pp, dec->b0, ACT_RELU});
-  XRD_GEMM({W, Pn, W, dec->w1, W, 0, ar(ra_h1()), Pp, ar(ra_h2()), Pp, dec->b1, ACT_RELU});
-  // sdf_out: torch row 0 = sdf, rows 1..128 = feat
-  XRD_GEMM({W, Pn, W, dec->ws + W, W, 0, ar(ra_h2()), Pp, ar(ra_feat()), Pp, dec->bs + 1, ACT_NONE});
-  XRD_GEMM({1, Pn, W, dec->ws, W, 0, ar(ra_h2()), Pp, Q.sdf, Pn, dec->bs, ACT_NONE});
-  // colour: relu(wc0 [feat, x] + bc0) -> sigmoid(wc1 . + bc1)
-  XRD_GEMM({W, Pn, W + EMB, dec->wc0, W + EMB, 0, ar(ra_feat()), Pp, ar(ra_c1()), Pp, dec->bc0, ACT_RELU});
-  XRD_GEMM({3, Pn, W, dec->wc1, W, 0, ar(ra_c1()), Pp, Q.rgb, Pn, dec->bc1, ACT_SIGMOID});
+  const int st = vox_forward(Q, dec, stream);
+  if (st != XRD_OK) return st;
   }
 
   RayParams Y;

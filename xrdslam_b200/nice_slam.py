@@ -13,6 +13,7 @@ import torch
 
 from .algorithm import Algorithm, AlgorithmConfig
 from .conv_onet import ConvOnetConfig
+from .mesher import MesherConfig
 from .optimizers import AdamOptimizerConfig
 from .schedulers import LRconfig, NiceSLAMSchedulerConfig
 
@@ -37,6 +38,7 @@ class NiceSLAMConfig(AlgorithmConfig):
     a coarse mapper runs after every mapping call, nice_slam.py:102-109)."""
     _target: Type = field(default_factory=lambda: NiceSLAM)
     model: ConvOnetConfig = field(default_factory=ConvOnetConfig)
+    mesher: MesherConfig = field(default_factory=MesherConfig)
     coarse: bool = True
     tracking_n_iters: int = 10
     mapping_n_iters: int = 60
@@ -71,6 +73,9 @@ class NiceSLAM(Algorithm):
         self.config.model.coarse = self.config.coarse
         self.model = self.config.model.setup(camera=camera, bounding_box=self.bounding_box)
         self.model.to(device)
+        self.mesher = self.config.mesher.setup(camera=camera, bounding_box=self.bounding_box,
+                                               marching_cubes_bound=self.marching_cube_bound)
+        self.cur_mesh = None
 
     # nice_slam.py:72-112
     def do_mapping(self, cur_frame):
@@ -169,3 +174,12 @@ class NiceSLAM(Algorithm):
     def render_img(self, c2w, gt_depth=None, idx=None):
         with self.lock, torch.no_grad():
             return self._render_full(c2w, gt_depth, extra={'stage': 'color'})
+
+    # nice_slam.py:281-288
+    def get_mesh(self):
+        with self.lock:
+            self.cur_mesh = self.mesher.get_mesh(keyframe_graph=self.keyframe_graph,
+                                                 query_fn=self.model.query_fn,
+                                                 color_func=self.model.color_func,
+                                                 device=self.device)
+            return self.cur_mesh

@@ -211,6 +211,41 @@ class SparseVoxel(Model):
     def get_map_states(self):
         return dict(self.map_states)
 
+    def octree_tables(self):
+        """voxels f32 [N,4], children f32 [N,8], features i32 [N,8] on the map's device."""
+        if self._dev_svo is not None:
+            return self._dev_svo.export()
+        return tuple(t.to(self.embeddings.device) for t in self.export_octree())
+
+    @torch.no_grad()
+    def query(self, points, voxel_ids, centres, vertex_idx):
+        """voxel_helpers_voxfusion.py:15-95 (get_scores / eval_points): decoder outputs
+        raw [P,4] = (rgb, sdf) at device points [P,3], each interpolated inside voxel
+        ``voxel_ids[p]`` -- a row of ``centres`` [N,3] / ``vertex_idx`` [N,8] (the mesher's
+        filtered voxel list)."""
+        dev = self.embeddings.device
+        P = points.shape[0]
+        raw = torch.empty(P, 4, dtype=torch.float32, device=dev)
+        if P == 0:
+            return raw
+        lib = _cabi.lib()
+        emb = self.embeddings.detach()
+        centres = centres.to(dev, torch.float32).contiguous()
+        vertex_idx = vertex_idx.to(dev, torch.int32).contiguous()
+        mp = XrdVoxMap(centres.shape[0], ptr(centres), None, ptr(vertex_idx), ptr(emb),
+                       emb.shape[0])
+        dec = _dec_struct([t.detach() for t in self.decoder.tensors()], XrdVoxDecoder)
+        pts = points.to(dev, torch.float32).contiguous()
+        ids = voxel_ids.to(dev, torch.int32).contiguous()
+        nb = lib.xrd_voxfusion_query_workspace_bytes(P)
+        ws = torch.empty(nb, dtype=torch.uint8, device=dev)
+        with torch.cuda.device(dev):
+            st = lib.xrd_voxfusion_query(C.byref(mp), C.byref(dec), self.config.voxel_size,
+                                         ptr(pts), ptr(ids), P, ptr(raw), ptr(ws), nb,
+                                         torch.cuda.current_stream(dev).cuda_stream)
+        check('xrd_voxfusion_query', st)
+        return raw
+
     # -------------------------------------------------------------- C-ABI ---
     def _map_struct(self, emb):
         ms = self.map_states
